@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — the IndexTTS-2.5 per-segment hot path on B200 (BASELINE.json configs[1]).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--quick] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one utterance through the whole per-segment pipeline of IndexTTS2.infer
@@ -152,6 +152,21 @@ def run_utterance(e, inp, prompt_emb, host: bool):
         res = e.codes_to_wav(dcodes, inp["pc_d"], inp["mel_d"], inp["style_d"], inp["z_d"], inp["F"],
                              CFM_STEPS, CFG_RATE, want_wav=False, want_pcm16=True)
     return codes, res["pcm16"]
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+PCM_SAMPLE = 1 << 20      # samples kept of a job's concatenated pcm16 (a whole config-5 job has ~1e8)
+
+
+def dump_outputs(out_dir, arrays):
+    """`--dump-outputs`: one DIR/<name>.npy per array, float32 or float64 (codes and pcm16 are integers, exact in
+    either), so that two builds of the project can be compared output for output on the same seeded inputs."""
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, f"dump of {total} bytes exceeds {DUMP_LIMIT_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def stage_breakdown(e):
@@ -314,19 +329,23 @@ def run_job(args, rank, world, local):
     if rank != 0:
         ge.build()
     e, cfg, wg, t_load = build_engine(local, max_batch=8)
-    line = job_line(args.workload, e, cfg, wg, dist, rank, world, local)
+    outputs = {} if args.dump_outputs else None
+    line = job_line(args.workload, e, cfg, wg, dist, rank, world, local, outputs)
     if rank == 0:
         print(json.dumps(line))
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
     if dist is not None:
         dist.destroy_process_group()
 
 
-def job_line(workload, e, cfg, wg, dist, rank, world, local):
+def job_line(workload, e, cfg, wg, dist, rank, world, local, outputs=None):
     """The whole fixed job once (after a warm-up mini-job), strong scaling over the ranks; returns the JSON line on rank 0.
     GPT decodes up to 8 utterances per group (sorted by length so a group's rows finish together; a row that reached its
     own length keeps decoding until the group's longest is done — those extra tokens are not counted); the tail runs
     per utterance.  Reports useful speech-tokens/s and RTF of the whole job, per-stage device time and the per-rank
-    busy time (LPT imbalance)."""
+    busy time (LPT imbalance).  `outputs` (a dict) receives this rank's results of the timed job: the codes of its
+    utterances in utterance order, concatenated, and a seeded sample of their concatenated pcm16."""
     from indextts_b200.sharding import broadcast_latents, gather_wavs, lpt_assign
     dev = torch.device("cuda", local)
     job = make_job(workload)
@@ -347,7 +366,7 @@ def job_line(workload, e, cfg, wg, dist, rank, world, local):
 
     def process(utts):
         t_g = t_c = t_v = 0.0
-        wavs, ntok = [], 0
+        wavs, kept, ntok = [], [], 0
         for g0 in range(0, len(utts), 8):
             grp = utts[g0:g0 + 8]
             prompts = [e.gpt_prepare_inputs(lats[u["spk"]]["style"], lats[u["spk"]]["emo"], texts[u["idx"]], 1) for u in grp]
@@ -365,8 +384,9 @@ def job_line(workload, e, cfg, wg, dist, rank, world, local):
                 t_c += e.s2mel_last_ms()["cfm_ms"]
                 t_v += e.bigvgan_last_ms()
                 wavs.append(res["pcm16"])
+                kept.append(codes[:n])
                 ntok += n
-        return wavs, ntok, (t_g, t_c, t_v)
+        return wavs, kept, ntok, (t_g, t_c, t_v)
 
     def barrier():
         e.sync()
@@ -382,7 +402,7 @@ def job_line(workload, e, cfg, wg, dist, rank, world, local):
     sampler.start()
     l0 = e.launches
     t0 = time.perf_counter()
-    wavs, ntok, (t_g, t_c, t_v) = process(mine)
+    wavs, kept, ntok, (t_g, t_c, t_v) = process(mine)
     e.sync()
     torch.cuda.synchronize()
     t_busy = time.perf_counter() - t0
@@ -392,6 +412,12 @@ def job_line(workload, e, cfg, wg, dist, rank, world, local):
     t_job = time.perf_counter() - t0
     clocks = sampler.stop()
     launches = e.launches - l0
+    if outputs is not None and mine:
+        order = sorted(range(len(mine)), key=lambda i: mine[i]["idx"])
+        pcm = torch.cat([wavs[i].reshape(-1) for i in order])
+        sel = np.sort(np.random.default_rng(0).integers(0, pcm.numel(), min(PCM_SAMPLE, pcm.numel())))
+        outputs["codes"] = np.concatenate([kept[i] for i in order]).astype(np.float64)
+        outputs["pcm16_sample"] = pcm[torch.from_numpy(sel).to(dev)].float().cpu().numpy()
     stats = torch.tensor([t_job, t_busy, t_g, t_c, t_v, float(ntok), float(launches)], device=dev, dtype=torch.float64)
     if dist is not None:
         allst = [torch.zeros_like(stats) for _ in range(world)]
@@ -431,7 +457,15 @@ def main():
     ap.add_argument("--no-config5", action="store_true", help="skip the config-5 job block of the default run")
     ap.add_argument("--workload", default="config2", choices=["config2", "config3", "config5"],
                     help="config2 (default): the batch-1 headline; config3 / config5: the fixed batch jobs, run once")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 / "
+                         "float64, <= 64 MB): codes and pcm16 of the headline utterance and, when it runs, codes and a "
+                         "seeded pcm16 sample of the batch job; rank 0's results")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what the B200 path computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -442,7 +476,7 @@ def main():
         run_job(args, rank, world, local)
         return
     W = max(3, args.warmup)
-    K = max(1, args.steps)
+    K = args.steps
 
     import __graft_entry__ as ge
     if rank == 0:
@@ -492,7 +526,7 @@ def main():
     g_ms = c_ms = v_ms = 0.0
     gpt_launch_ms, gpt_launches = 0.0, 0
     for _ in range(K):
-        run_utterance(e, mine, prompt_emb_d, host=False)
+        codes, pcm = run_utterance(e, mine, prompt_emb_d, host=False)
         g, s = stage_breakdown(e)
         g_ms += g["prefill_ms"] + g["decode_ms"]
         gpt_launch_ms += g["decode_ms"]
@@ -504,6 +538,7 @@ def main():
     clocks = sampler.stop()
     t_dev = e.event_elapsed_ms(0, 1) / 1000.0
     launches = e.launches - l0
+    outputs = {"codes": codes.astype(np.float64), "pcm16": pcm.float().cpu().numpy()} if args.dump_outputs else None
     # ---- end to end: host buffers in, pcm16 out, gather on rank 0 ----
     if dist is not None:
         from indextts_b200.sharding import gather_wavs
@@ -534,7 +569,10 @@ def main():
     # after the timed regions of the headline: reported as an extra block, the headline stays config 2 (VERDICT r1 item 6)
     job5 = None
     if not args.no_config5:
-        job5 = job_line("config5", e, cfg, wg, dist, rank, world, local)
+        job_out = {} if outputs is not None else None
+        job5 = job_line("config5", e, cfg, wg, dist, rank, world, local, job_out)
+        if job_out:
+            outputs.update({"config5_" + k: v for k, v in job_out.items()})
     if rank != 0:
         if dist is not None:
             dist.destroy_process_group()
@@ -592,6 +630,8 @@ def main():
             line["cpu_baseline"] = {"value": None, "unit": "tokens/s", "cores": os.cpu_count(), "kind": "port",
                                     "sample": f"failed: {ex}"}
     print(json.dumps(line))
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if dist is not None:
         dist.destroy_process_group()
 

@@ -1,16 +1,63 @@
-"""CPU (build container only: needs /root/reference): `dropin.load_reference_weights` against the REAL reference
-modules.  The reference's own classes are instantiated (random init, small dims) through oracle/refimport.py, a
-recording stand-in replaces the engine, and the test checks that every hyper-parameter the drop-in derives from the
-modules' state dicts equals what the modules were constructed with, and that every tensor name the engine will ask for
-(`gpt.…`, `s2mel.…`, `codec.…`, `bigvgan.…`) is present.  Skipped where the reference tree is absent (GPU box)."""
+"""CPU: `dropin.load_reference_weights` / `attach` / `attach_v1` against the reference's own modules and call sites, as
+recorded in tests/golden/reference_interfaces.json (oracle/make_goldens_interfaces.py): for small modules built by the
+reference's own classes, the name / shape / dtype of every state-dict entry and the plain attributes the drop-in reads;
+and every call `infer_v2_5.py` / `infer.py` make at the rebound seams.  Stand-ins rebuilt from the record go through the
+drop-in, a recording stand-in replaces the engine, and the test checks that every hyper-parameter the drop-in derives
+from the state dicts equals what the modules were constructed with, that every tensor name the engine will ask for
+(`gpt.…`, `s2mel.…`, `codec.…`, `bigvgan.…`) is present, and that the reference's calls bind to the rebound seams."""
+import json
+import os
 import types
 
-import pytest
 import torch
 
-from oracle import refimport
+GOLD = os.path.join(os.path.dirname(__file__), "golden", "reference_interfaces.json")
 
-pytestmark = pytest.mark.skipif(not refimport.available(), reason="/root/reference not present")
+
+def _golden():
+    with open(GOLD) as f:
+        return json.load(f)
+
+
+def _module(rec):
+    """Stand-in for a recorded reference module: its state dict, placeholder values under the reference's names,
+    shapes and dtypes."""
+    sd = {k: torch.ones(shape, dtype=getattr(torch, dt)) for k, (shape, dt) in rec["state_dict"].items()}
+    return types.SimpleNamespace(state_dict=lambda: sd)
+
+
+def _gpt(rec):
+    """Stand-in for a reference `UnifiedVoice` (v2 or v1) with the attributes the drop-in reads."""
+    a = rec["attrs"]
+    m = _module(rec)
+    m.gpt = types.SimpleNamespace(h=[None] * a["blocks"])
+    for k in ("model_dim", "heads", "number_mel_codes", "start_mel_token", "stop_mel_token", "max_mel_tokens"):
+        setattr(m, k, a[k])
+    if a.get("emo_input_size") is not None:
+        m.emo_input_size = a["emo_input_size"]
+    if "emo_perceiver_encoder.latents" in m.state_dict():
+        m.emo_perceiver_encoder = types.SimpleNamespace(latents=m.state_dict()["emo_perceiver_encoder.latents"])
+        if a.get("emo_perceiver_heads") is not None:
+            m.emo_perceiver_encoder.heads = a["emo_perceiver_heads"]
+    if "kv_cache" in a:
+        m.inference_model = types.SimpleNamespace(kv_cache=a["kv_cache"])
+    return m
+
+
+def _bigvgan(rec):
+    m = _module(rec)
+    m.h = rec["h"]
+    return m
+
+
+def _reference_tts():
+    """The modules of a reference IndexTTS2 (infer_v2_5) that `attach` reads and rebinds."""
+    mods = _golden()["modules"]
+    s2 = _module(mods["s2mel"])
+    s2.models = {name: types.SimpleNamespace() for name in mods["s2mel"]["models"]}
+    s2.models["cfm"].in_channels = mods["s2mel"]["attrs"]["cfm_in_channels"]
+    return types.SimpleNamespace(gpt=_gpt(mods["gpt"]), s2mel=s2, semantic_codec=_module(mods["semantic_codec"]),
+                                 bigvgan=_bigvgan(mods["bigvgan"]))
 
 
 class RecordingEngine:
@@ -43,19 +90,12 @@ class RecordingEngine:
 def test_config_derivation_from_real_reference_modules():
     from indextts_b200 import synth
     from indextts_b200.dropin import load_reference_weights
-    from oracle.gpt import make_gpt_weights
     from oracle.validate_gpt_vs_hf import small_case
 
     cfg, _, _, _ = small_case()
-    cfg = dict(cfg, n_langs=106)
-    gpt = refimport.gpt_module(cfg, make_gpt_weights(cfg, seed=1, bf16=False))
-    s2 = refimport.s2mel_module(refimport.s2mel_args(hidden=64, heads=1, depth=3, wn_hidden=64, wn_layers=2,
-                                                     content_dim=64, lr_in=96, style_dim=24))
-    codec = refimport.codec_module(codebook_size=64, hidden_size=96, codebook_dim=8, vocos_dim=48,
-                                   vocos_intermediate_dim=64, vocos_num_layers=2)
     h = synth.small_config()
-    bv = refimport.bigvgan_module(h)
-    tts = types.SimpleNamespace(gpt=gpt, s2mel=s2, semantic_codec=codec, bigvgan=bv)
+    tts = _reference_tts()
+    gpt = tts.gpt
     eng = RecordingEngine()
     load_reference_weights(eng, tts, max_batch=4)
 
@@ -88,52 +128,22 @@ def test_config_derivation_from_real_reference_modules():
         "weight-norm pairs must be folded before they reach the engine"
 
 
-def _reference_call_sites():
-    """(positional count, keyword names) of the calls `infer_generator` makes at the six seams (infer_v2_5.py:749-864),
-    read from the reference source with ast."""
-    import ast
-    import os
-    src = open(os.path.join(refimport.REF, "indextts", "infer_v2_5.py")).read()
-    tree = ast.parse(src)
-    want = {"self.gpt.merge_emovec": "merge_emovec", "self.gpt.inference_speech": "inference_speech",
-            "self.semantic_codec.decode": "codec_decode", "self.s2mel.models['length_regulator']": "length_regulator",
-            "self.s2mel.models['cfm'].inference": "cfm_inference", "self.bigvgan": "bigvgan"}
-    found = {}
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call):
-            name = ast.unparse(node.func)
-            if name in want:
-                kws = [k.arg for k in node.keywords if k.arg is not None]
-                star = any(k.arg is None for k in node.keywords)
-                found.setdefault(want[name], []).append((len(node.args), kws, star))
-    return found
-
-
 def test_rebound_seams_accept_the_reference_call_sites():
     """Every call `infer_v2_5.py` makes at a seam binds to the callable `attach` installs there (same positional
-    arity, same keyword names) — the drop-in claim of INTEGRATION.md, checked against the reference source."""
+    arity, same keyword names) — the drop-in claim of INTEGRATION.md, checked against the reference's call sites
+    ((positional count, keyword names, **kwargs passed) per call, read from its source with ast)."""
     import inspect
 
-    from indextts_b200 import synth
     from indextts_b200.dropin import attach
-    from oracle.gpt import make_gpt_weights
-    from oracle.validate_gpt_vs_hf import small_case
 
-    cfg, _, _, _ = small_case()
-    cfg = dict(cfg, n_langs=106)
-    gpt = refimport.gpt_module(cfg, make_gpt_weights(cfg, seed=1, bf16=False))
-    s2 = refimport.s2mel_module(refimport.s2mel_args(hidden=64, heads=1, depth=3, wn_hidden=64, wn_layers=2,
-                                                     content_dim=64, lr_in=96, style_dim=24))
-    codec = refimport.codec_module(codebook_size=64, hidden_size=96, codebook_dim=8, vocos_dim=48,
-                                   vocos_intermediate_dim=64, vocos_num_layers=2)
-    bv = refimport.bigvgan_module(synth.small_config())
-    tts = types.SimpleNamespace(gpt=gpt, s2mel=s2, semantic_codec=codec, bigvgan=bv)
+    tts = _reference_tts()
+    gpt, bv = tts.gpt, tts.bigvgan
     eng = RecordingEngine()
     attach(tts, engine=eng)
     seams = {"merge_emovec": tts.gpt.merge_emovec, "inference_speech": tts.gpt.inference_speech,
              "codec_decode": tts.semantic_codec.decode, "length_regulator": tts.s2mel.models["length_regulator"].forward,
              "cfm_inference": tts.s2mel.models["cfm"].inference, "bigvgan": tts.bigvgan.forward}
-    sites = _reference_call_sites()
+    sites = _golden()["call_sites"]["infer_v2_5"]
     assert set(sites) == set(seams), (sorted(sites), sorted(seams))
     for name, calls in sites.items():
         sig = inspect.signature(seams[name])
@@ -150,20 +160,17 @@ def test_attach_v1_on_real_reference_v1_modules():
     """v1 / v1.5 drop-in (row a13): `attach_v1` on the reference's own v1 `UnifiedVoice` and `BigVGAN` classes — the derived
     prompt-encoder / vocoder configuration equals what the modules were built with, and the calls `indextts/infer.py` makes
     at the three seams bind to the rebound callables."""
-    import ast
     import inspect
-    import os
 
     from indextts_b200 import synth
     from indextts_b200.dropin import attach_v1
-    from oracle.make_goldens_v1 import reference_module
     from oracle.validate_gpt_vs_hf import small_case
 
     cfg, _, _, _ = small_case()
     ccfg = synth.small_v1_cond_cfg(cfg["model_dim"])
-    gpt = refimport.gpt_module_v1(cfg, ccfg, synth.make_gpt_v1_weights(cfg, ccfg, seed=3), kv_cache=False)
     h = synth.small_v1_config()
-    bv = reference_module(h, synth.make_bigvgan_v1_weights(h, seed=5))
+    doc = _golden()
+    gpt, bv = _gpt(doc["modules"]["v1_gpt"]), _bigvgan(doc["modules"]["v1_bigvgan"])
     tts = types.SimpleNamespace(gpt=gpt, bigvgan=bv)
 
     class Rec(RecordingEngine):
@@ -185,13 +192,9 @@ def test_attach_v1_on_real_reference_v1_modules():
     assert "bigvgan_v1.speaker_encoder.blocks.0.conv.conv.weight" in eng.weights and "bigvgan_v1.cond_layer.weight" in eng.weights
     assert "gpt.conditioning_encoder.embed.out.0.weight" in eng.weights and "gpt.perceiver_encoder.latents" in eng.weights
     # call sites of indextts/infer.py
-    tree = ast.parse(open(os.path.join(refimport.REF, "indextts", "infer.py")).read())
     want = {"self.gpt.inference_speech": tts.gpt.inference_speech, "self.gpt": tts.gpt.forward, "self.bigvgan": tts.bigvgan.forward}
-    seen = set()
-    for node in ast.walk(tree):
-        if isinstance(node, ast.Call) and ast.unparse(node.func) in want:
-            name = ast.unparse(node.func)
-            kws = [k.arg for k in node.keywords if k.arg is not None]
-            inspect.signature(want[name]).bind(*([None] * len(node.args)), **{k: None for k in kws})
-            seen.add(name)
-    assert seen == set(want)
+    sites = doc["call_sites"]["infer"]
+    assert set(sites) == set(want)
+    for name, calls in sites.items():
+        for npos, kws, _star in calls:
+            inspect.signature(want[name]).bind(*([None] * npos), **{k: None for k in kws})
