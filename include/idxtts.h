@@ -292,6 +292,29 @@ int idx_debug_conv_gemm(idx_engine* e, const float* A, int B, int Tin, int K, co
                         int ldo, long long out_valid, long long out_elems_per_batch, int backend,
                         float* out);
 
+/* Diagnostic (tests): the fp16 tensor-core GEMM of idx_debug_conv_gemm with a fused pair epilogue, its operands
+ * prepared as the DiT / WaveNet prepare them (fp16 images of A and wk; SwiGLU / gate weight rows and bias interleaved).
+ * wk [N][taps*K] and bias [N] (or null) in the module's row order; fp16 results as raw bits:
+ *   epi 1 (SwiGLU): rows w1 | w3  -> out16 [B][M][N/2] = silu(w1 x + b1) * (w3 x + b3)
+ *   epi 2 (gate):   rows a | c    -> out16 [B][M][N/2] = tanh(a + g[b][j]) * sigmoid(c + g[b][N/2 + j]),
+ *                   g = aux [B][aux_stride] (aux_stride 0: one [N] vector for every batch entry)
+ *   epi 3 (RoPE):   rows q | k | v of H = aux_stride heads of 64 (N = 192 H), RoPE table over T = M rows (aux unused)
+ *                   -> out16 = Qr | Kr | Vb, each [B*H][M][64]: q rotated and multiplied by scale, k rotated, v as is.
+ * N % 32 != 0 or a missing gate vector returns IDX_ERR_ARG.                                                    */
+int idx_debug_gemm_pair_epilogue(idx_engine* e, const float* A, int B, int Tin, int K, const float* wk,
+                                 int taps, int dil, int pad, int M, int N, const float* bias, int epi,
+                                 const float* aux, int aux_stride, float scale, uint16_t* out16);
+
+/* Diagnostic (tests): flash attention over fp16 qkv16 = Qr | Kr | Vb, each [B*H][T][64] (what epi 3 above writes),
+ * through kernel 1 (mma.sync; q pre-scaled by 1/8, softmax in base e) or 2 (tcgen05; q pre-scaled by log2(e)/8,
+ * softmax in base 2).  out [B][T][H*64] f32 and / or out16 (fp16 bits, same shape); either may be null.          */
+int idx_debug_flash_attention(idx_engine* e, const uint16_t* qkv16, int B, int T, int H, int kernel,
+                              float* out, uint16_t* out16);
+
+/* Diagnostic (tests): the DiT attention with interleaved-pair RoPE (base 1e4) on fp32 qkv [B][T][3*H*64] (q | k | v)
+ * -> out [B][T][H*64] through backend 1 (SIMT fp32) or 0 (fp16 rotate / split + mma.sync flash kernel).           */
+int idx_debug_attention_rope(idx_engine* e, const float* qkv, int B, int T, int H, int backend, float* out);
+
 /* ---------------------------------------------------------------- s2mel + codec -- */
 
 /* Geometry of the s2mel section of config.yaml as MyModel reads it

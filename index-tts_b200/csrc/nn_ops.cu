@@ -681,8 +681,7 @@ void attention_rope(idx_engine* e, const float* qkv, float* out, int B, int T, i
     __half* Vb = (__half*)e->arena.alloc((size_t)BH * T * AD * 2);
     launch_pdl(e, rope_split_fa_kernel, dim3(T, H, B), dim3(AD), 0, qkv, rope, Qr, Kr, Vb, T, H);
     LAUNCH_CHECK(e);
-    launch_pdl(e, flash_attn_tc_kernel, dim3((T + FQ - 1) / FQ, (unsigned)BH), dim3(128), 0, (const __half*)Qr, (const __half*)Kr, (const __half*)Vb, out, T, H, out16);
-    LAUNCH_CHECK(e);
+    flash_attention_mma(e, Qr, Kr, Vb, out, out16, B, T, H);
     e->arena.off = mark;
     return;
   }
@@ -729,14 +728,73 @@ static bool fa5_on() {
   return on;
 }
 float flash_attention_q_scale() { return fa5_on() ? 0.125f * 1.4426950408889634f : 0.125f; }
+void flash_attention_mma(idx_engine* e, const __half* Qr, const __half* Kr, const __half* Vb, float* out, __half* out16,
+                         int B, int T, int H) {
+  launch_pdl(e, flash_attn_tc_kernel, dim3((T + FQ - 1) / FQ, (unsigned)((long long)B * H)), dim3(128), 0, Qr, Kr, Vb, out, T, H, out16);
+  LAUNCH_CHECK(e);
+}
 void flash_attention_split(idx_engine* e, const __half* Qr, const __half* Kr, const __half* Vb, float* out, __half* out16,
                            int B, int T, int H) {
   if (fa5_on()) {
     flash_attention_tc5(e, Qr, Kr, Vb, out, out16, B, T, H);
     return;
   }
-  launch_pdl(e, flash_attn_tc_kernel, dim3((T + FQ - 1) / FQ, (unsigned)((long long)B * H)), dim3(128), 0, Qr, Kr, Vb, out, T, H, out16);
-  LAUNCH_CHECK(e);
+  flash_attention_mma(e, Qr, Kr, Vb, out, out16, B, T, H);
+}
+
+// Diagnostic entry (tests): one flash attention over fp16 Qr | Kr | Vb [B*H][T][64] (what EPI_ROPE writes) through the
+// chosen kernel: 1 = flash_attn_tc_kernel (mma.sync, scores in base e), 2 = fa5_kernel (tcgen05, scores in base 2).
+extern "C" int idx_debug_flash_attention(idx_engine* e, const uint16_t* qkv16, int B, int T, int H, int kernel, float* out,
+                                         uint16_t* out16) {
+  IDX_API_BEGIN
+  IDX_CHECK(e && qkv16 && (out || out16), IDX_ERR_ARG, "null argument");
+  IDX_CHECK(B > 0 && T > 0 && H > 0, IDX_ERR_ARG, "idx_debug_flash_attention: B, T, H must be positive");
+  IDX_CHECK(kernel == 1 || kernel == 2, IDX_ERR_ARG, "idx_debug_flash_attention: kernel 1 = mma.sync, 2 = tcgen05");
+  IDX_CUDA(cudaSetDevice(e->device));
+  const size_t n = (size_t)B * H * T * AD;       // elements of one of Qr / Kr / Vb, and of the output
+  e->ensure_arena(2 * 3 * n + 4 * n + 2 * n + (4 << 10));
+  e->arena.reset();
+  __half* d_qkv = e->arena.get<__half>(3 * n);
+  float* d_out = out ? e->arena.get<float>(n) : nullptr;
+  __half* d_out16 = out16 ? e->arena.get<__half>(n) : nullptr;
+  idx_to_device(e, d_qkv, qkv16, 3 * n * 2);
+  if (kernel == 1) flash_attention_mma(e, d_qkv, d_qkv + n, d_qkv + 2 * n, d_out, d_out16, B, T, H);
+  else flash_attention_tc5(e, d_qkv, d_qkv + n, d_qkv + 2 * n, d_out, d_out16, B, T, H);
+  if (out) idx_from_device(e, out, d_out, n * 4);
+  if (out16) idx_from_device(e, out16, d_out16, n * 2);
+  IDX_CUDA(cudaStreamSynchronize(e->stream));
+  IDX_API_END(e)
+}
+
+// Diagnostic entry (tests): attention_rope on fp32 qkv [B][T][3*H*64] with the RoPE table of the DiT; backend 1 = the SIMT
+// fp32 attention_kernel (strict path), 0 = rope_split_fa_kernel + the mma.sync flash kernel (tf32-tail path).
+extern "C" int idx_debug_attention_rope(idx_engine* e, const float* qkv, int B, int T, int H, int backend, float* out) {
+  IDX_API_BEGIN
+  IDX_CHECK(e && qkv && out, IDX_ERR_ARG, "null argument");
+  IDX_CHECK(B > 0 && T > 0 && H > 0, IDX_ERR_ARG, "idx_debug_attention_rope: B, T, H must be positive");
+  IDX_CHECK(backend == 0 || backend == 1, IDX_ERR_ARG, "idx_debug_attention_rope: backend 0 = tensor cores, 1 = SIMT fp32");
+  IDX_CUDA(cudaSetDevice(e->device));
+  const size_t nq = (size_t)B * T * 3 * H * AD, no = (size_t)B * T * H * AD, nt = (size_t)T * AD;
+  // attention_rope's tensor-core path allocates Qr | Kr | Vb fp16 from the arena after these
+  e->ensure_arena(4 * (nq + no + nt) + 2 * 3 * no + (8 << 10));
+  e->arena.reset();
+  float* d_qkv = e->arena.get<float>(nq);
+  float* d_out = e->arena.get<float>(no);
+  float* d_rope = e->arena.get<float>(nt);
+  idx_to_device(e, d_qkv, qkv, nq * 4);
+  rope_table(e, d_rope, T, AD);
+  const int saved = e->gemm_backend;
+  e->gemm_backend = backend;
+  try {
+    attention_rope(e, d_qkv, d_out, B, T, H, d_rope, nullptr);
+  } catch (...) {
+    e->gemm_backend = saved;
+    throw;
+  }
+  e->gemm_backend = saved;
+  idx_from_device(e, out, d_out, no * 4);
+  IDX_CUDA(cudaStreamSynchronize(e->stream));
+  IDX_API_END(e)
 }
 void cfg_euler(idx_engine* e, float* x, const float* v_cond, const float* v_uncond, float dt, float rate, int T,
                int C, int P) {

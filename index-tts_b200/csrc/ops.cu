@@ -411,3 +411,66 @@ extern "C" int idx_debug_conv_gemm(idx_engine* e, const float* A, int B, int Tin
   IDX_CUDA(cudaStreamSynchronize(e->stream));
   IDX_API_END(e)
 }
+
+// Diagnostic entry (tests): one fp16 tensor-core GEMM with a fused pair epilogue, prepared the way the DiT / WaveNet
+// prepare theirs: fp16 images by to_half, SwiGLU / gate weights and bias interleaved by pack_half_interleaved, the RoPE
+// table by rope_table.  wk [N][taps*K] and bias [N] are in the module's row order (w1 | w3, a | c, q | k | v).
+extern "C" int idx_debug_gemm_pair_epilogue(idx_engine* e, const float* A, int B, int Tin, int K, const float* wk, int taps,
+                                            int dil, int pad, int M, int N, const float* bias, int epi, const float* aux,
+                                            int aux_stride, float scale, uint16_t* out16) {
+  IDX_API_BEGIN
+  IDX_CHECK(e && A && wk && out16, IDX_ERR_ARG, "null argument");
+  IDX_CHECK(B > 0 && Tin > 0 && K > 0 && taps > 0 && M > 0 && N > 0, IDX_ERR_ARG, "idx_debug_gemm_pair_epilogue: bad sizes");
+  IDX_CHECK(epi == EPI_SWIGLU || epi == EPI_WNGATE || epi == EPI_ROPE, IDX_ERR_ARG,
+            "idx_debug_gemm_pair_epilogue: epi 1 = SwiGLU, 2 = WaveNet gate, 3 = RoPE");
+  if (epi == EPI_ROPE)
+    IDX_CHECK(aux_stride > 0 && N == 3 * 64 * aux_stride, IDX_ERR_ARG, "EPI_ROPE: N must be 3 * 64 * heads (aux_stride = heads)");
+  if (epi == EPI_WNGATE)
+    IDX_CHECK(aux && (aux_stride == 0 || aux_stride >= N), IDX_ERR_ARG,
+              "EPI_WNGATE: needs the gate g [N] (aux_stride 0: shared by every batch entry) or [B][aux_stride >= N]");
+  IDX_CUDA(cudaSetDevice(e->device));
+  const size_t na = (size_t)B * Tin * K, nw = (size_t)N * taps * K;
+  const size_t no = (epi == EPI_ROPE) ? (size_t)B * M * N : (size_t)B * M * (N / 2);
+  const size_t ng = (epi == EPI_WNGATE) ? (size_t)(B - 1) * aux_stride + N : 0;
+  const size_t nt = (epi == EPI_ROPE) ? (size_t)M * 64 : 0;
+  e->ensure_arena(4 * (na + nw + N + ng + nt) + 2 * (na + nw + no) + (8 << 10));
+  e->arena.reset();
+  float* dA = e->arena.get<float>(na);
+  float* dWk = e->arena.get<float>(nw);
+  float* dBias = bias ? e->arena.get<float>(N) : nullptr;
+  __half* dA16 = e->arena.get<__half>(na);
+  __half* dOut = e->arena.get<__half>(no);
+  idx_to_device(e, dA, A, na * 4);
+  idx_to_device(e, dWk, wk, nw * 4);
+  if (bias) idx_to_device(e, dBias, bias, (size_t)N * 4);
+  to_half(e, dA, dA16, (long long)na);
+  ConvGemm g;
+  g.A16 = dA16; g.B = B; g.Tin = Tin; g.K = K; g.taps = taps; g.dil = dil; g.pad = pad; g.M = M; g.N = N;
+  g.epi = epi; g.out16 = dOut; g.aux_stride = aux_stride; g.scale = scale;
+  struct PoolGuard {           // the interleaved weights live outside the arena, like the model's
+    WeightPool p;
+    ~PoolGuard() { cudaDeviceSynchronize(); p.release(); }
+  } pool;
+  if (epi == EPI_ROPE) {
+    __half* dW16 = e->arena.get<__half>(nw);
+    to_half(e, dWk, dW16, (long long)nw);
+    float* tab = e->arena.get<float>(nt);
+    rope_table(e, tab, M, 64);
+    g.Wk16 = dW16; g.bias = dBias; g.aux = tab;
+  } else {
+    PackedW w;
+    w.wk = dWk; w.N = N; w.K = K; w.taps = taps; w.dil = dil; w.bias = dBias;
+    float* bias_i = nullptr;
+    g.Wk16 = pack_half_interleaved(e, pool.p, w, &bias_i);
+    g.bias = bias_i;
+    if (epi == EPI_WNGATE) {
+      float* dG = e->arena.get<float>(ng);
+      idx_to_device(e, dG, aux, ng * 4);
+      g.aux = dG;
+    }
+  }
+  conv_gemm(e, g);
+  idx_from_device(e, out16, dOut, no * 2);
+  IDX_CUDA(cudaStreamSynchronize(e->stream));
+  IDX_API_END(e)
+}

@@ -158,6 +158,9 @@ void flash_attention_split(idx_engine* e, const __half* Qr, const __half* Kr, co
                            int B, int T, int H);
 // scale EPI_ROPE must apply to q for flash_attention_split: 1/8, times log2(e) when the tcgen05 kernel (exp2 softmax) is on
 float flash_attention_q_scale();
+// the same on mma.sync (nn_ops.cu: flash_attn_tc_kernel, scores in base e: q pre-scaled by 1/8 only)
+void flash_attention_mma(idx_engine* e, const __half* Qr, const __half* Kr, const __half* Vb, float* out, __half* out16,
+                         int B, int T, int H);
 // the same on tcgen05 (gemm_tc.cu: S and O in tensor memory, P fed back as a tensor-memory operand)
 void flash_attention_tc5(idx_engine* e, const __half* Qr, const __half* Kr, const __half* Vb, float* out, __half* out16,
                          int B, int T, int H);

@@ -153,6 +153,12 @@ def load_library(path: str = None):
     lib.idx_debug_conv_gemm.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int,
                                         C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int,
                                         C.c_float, C.c_longlong, C.c_int, C.c_longlong, C.c_longlong, C.c_int, C.c_void_p]
+    lib.idx_debug_gemm_pair_epilogue.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int,
+                                                 C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p,
+                                                 C.c_int, C.c_float, C.c_void_p]
+    lib.idx_debug_flash_attention.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                              C.c_void_p]
+    lib.idx_debug_attention_rope.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p]
     lib.idx_s2mel_init.argtypes = [C.c_void_p, C.POINTER(S2melConfig)]
     lib.idx_codec_init.argtypes = [C.c_void_p, C.POINTER(CodecConfig)]
     lib.idx_codec_decode.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
@@ -600,6 +606,49 @@ class Engine:
                                                  biasN, act, _ptr(r_), int(accum), float(scale), int(out_off), ldo,
                                                  int(out_valid), int(per), int(backend), _ptr(out)),
                     "idx_debug_conv_gemm")
+        return out
+
+    def debug_gemm_pair_epilogue(self, A, wk, epi, taps=1, dil=1, pad=0, M=None, bias=None, aux=None, aux_stride=0,
+                                 scale=1.0):
+        """fp16 tensor-core GEMM with a fused pair epilogue (1 SwiGLU, 2 WaveNet gate, 3 RoPE; aux_stride = heads).
+        A [B][Tin][K] and wk [N][taps*K] in fp32, module row order.  Returns float16: [B][M][N/2] for epi 1 / 2, and
+        Qr | Kr | Vb as [3][B*H][M][64] for epi 3."""
+        A = np.ascontiguousarray(A, dtype=np.float32)
+        wk = np.ascontiguousarray(wk, dtype=np.float32)
+        B, Tin, K = A.shape
+        N = wk.shape[0]
+        M = Tin if M is None else M
+        b_ = None if bias is None else np.ascontiguousarray(bias, dtype=np.float32)
+        g_ = None if aux is None else np.ascontiguousarray(aux, dtype=np.float32)
+        if epi == 3:
+            H = max(int(aux_stride), 1)
+            out = np.zeros((3, B * H, M, 64), np.float16) if N == 192 * H else np.zeros(B * M * N, np.float16)
+        else:
+            out = np.zeros((B, M, max(N // 2, 1)), np.float16)
+        self._check(self.lib.idx_debug_gemm_pair_epilogue(self.h, _ptr(A), B, Tin, K, _ptr(wk), taps, dil, pad, M, N,
+                                                          _ptr(b_), int(epi), _ptr(g_), int(aux_stride), float(scale),
+                                                          _ptr(out)),
+                    "idx_debug_gemm_pair_epilogue")
+        return out
+
+    def debug_flash_attention(self, qkv16, B, T, H, kernel, want_out=True, want_out16=True):
+        """Flash attention on fp16 Qr | Kr | Vb ([3][B*H][T][64]) through kernel 1 (mma.sync) or 2 (tcgen05).
+        Returns (out f32 [B][T][H*64] or None, out16 float16 [B][T][H*64] or None)."""
+        q = np.ascontiguousarray(qkv16, dtype=np.float16)
+        assert q.size == 3 * B * H * T * 64
+        out = np.zeros((B, T, H * 64), np.float32) if want_out else None
+        out16 = np.zeros((B, T, H * 64), np.float16) if want_out16 else None
+        self._check(self.lib.idx_debug_flash_attention(self.h, _ptr(q), B, T, H, int(kernel), _ptr(out), _ptr(out16)),
+                    "idx_debug_flash_attention")
+        return out, out16
+
+    def debug_attention_rope(self, qkv, H, backend):
+        """The DiT attention with RoPE on fp32 qkv [B][T][3*H*64]: backend 1 SIMT fp32, 0 fp16 mma.sync flash."""
+        qkv = np.ascontiguousarray(qkv, dtype=np.float32)
+        B, T, _ = qkv.shape
+        out = np.zeros((B, T, H * 64), np.float32)
+        self._check(self.lib.idx_debug_attention_rope(self.h, _ptr(qkv), B, T, H, int(backend), _ptr(out)),
+                    "idx_debug_attention_rope")
         return out
 
     # ------------------------------------------------------------------- emotion --
